@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W             # our arm (one rank per GPU; torchrun for N > 1)
     python bench.py --impl reference --gpus N --steps K ...   # the reference's own CPU path on the host cores
     python bench.py --config 4                                # another BASELINE config as the headline line
+    python bench.py --dump-outputs DIR                        # also write the last timed step's results to DIR/*.npy
 
 Headline (default, `--config 2`): fused-elementwise GB/s on the fp64 arange/sin/cos/mul/add chain
 (sample/test-ramba.py:12-19 of the reference), 1e9 elements per GPU (weak scaling), a step =
@@ -22,11 +23,13 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the tree as it found it (it may be read-only)
 
 
 def parse():
@@ -44,7 +47,13 @@ def parse():
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--no-cpu", action="store_true")
     p.add_argument("--no-extra", action="store_true", help="skip configs 3-5 and the strong-scaling leg")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write the headline workload's results of its last step as DIR/<name>.npy "
+                        "(outputs larger than %d MiB in all: a fixed, seeded sample)" % (DUMP_BYTES >> 20))
+    args = p.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        p.error("--dump-outputs writes the results of --impl ours")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------
@@ -173,7 +182,9 @@ def run_reference_process(config, n, steps, warmup, threads, timeout=1500):
         env.pop(k, None)
     cmd = [sys.executable, os.path.join(ROOT, "oracle", "ref_runner.py"), "--config", str(config), "--n", str(int(n)),
            "--steps", str(steps), "--warmup", str(warmup)]
-    out = subprocess.run(cmd, env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=timeout)
+    with tempfile.TemporaryDirectory(prefix="rb200-numba-") as cache:  # the reference's Numba cache, not next to its sources
+        env.update({"NUMBA_CACHE_DIR": cache, "PYTHONDONTWRITEBYTECODE": "1"})
+        out = subprocess.run(cmd, env=env, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True, timeout=timeout)
     for line in reversed(out.stdout.strip().splitlines()):
         if line.startswith("{"):
             return json.loads(line)
@@ -348,6 +359,10 @@ class Chain:
         d = D[0:4096].asarray()
         return bool(np.max(np.abs(d - 1.0)) <= 4 * np.finfo(np.float64).eps)
 
+    def outputs(self):
+        B, C, D = self.out
+        return {"B": B, "C": C, "D": D}
+
     def describe(self):
         return {"elements_per_gpu": self.N // self.W, "global_elements": self.N, "bytes_per_element": 32}
 
@@ -379,6 +394,9 @@ class AffineSum:
 
     def check(self):
         return self.out == self.expect
+
+    def outputs(self):
+        return {"sum": self.out}
 
     def describe(self):
         return {"shape": [self.n, self.n], "bytes_per_element": 4}
@@ -428,6 +446,9 @@ class Laplacian:
         # the host at 1024^3; the full-array equality is in tests/test_baseline_sizes.py
         return ok
 
+    def outputs(self):
+        return {"V": self.V}
+
     def describe(self):
         return {"shape": [self.m] * 3, "bytes_per_element": 8}
 
@@ -461,11 +482,50 @@ class BcastAxisSum:
 
         return bool(np.array_equal(self.out.asarray(), self.expect))
 
+    def outputs(self):
+        return {"colsum": self.out}
+
     def describe(self):
         return {"shape": [self.r, self.c], "bytes_per_element": 4}
 
 
 CLASSES = {2: Chain, 3: AffineSum, 4: Laplacian, 5: BcastAxisSum}
+DUMP_BYTES = 48 << 20  # --dump-outputs: all files together
+
+
+def host_sample(a, budget, rng):
+    """`a` (an array of ramba_b200 or NumPy, or a scalar) on the host: whole when it takes at most `budget` bytes, else
+    contiguous blocks along axis 0 at positions drawn from `rng`, flattened.  Same shape, budget and rng state: same
+    positions, whatever computed `a` (asarray is collective, so every rank draws and reads the same)."""
+    import numpy as np
+
+    def host(x):
+        return x.asarray() if hasattr(x, "asarray") else np.asarray(x)
+
+    itemsize = np.dtype(a.dtype).itemsize if hasattr(a, "dtype") else 8
+    if np.ndim(a) == 0 or a.size * itemsize <= budget:
+        return host(a)
+    n0 = a.shape[0]
+    row = a.size // n0 * itemsize
+    if row > budget:
+        return host_sample(a[int(rng.integers(n0))], budget, rng)
+    blocks = min(64, budget // row)
+    rows = budget // row // blocks
+    starts = np.sort(rng.choice(n0 // rows, blocks, replace=False)) * rows
+    return np.concatenate([host(a[int(s):int(s) + rows]).ravel() for s in starts])
+
+
+def dump_outputs(wl, path, rank):
+    """`--dump-outputs`: the workload's results as `path`/<name>.npy, so that two builds can be compared output by output."""
+    import numpy as np
+
+    outs = wl.outputs()  # (one seed for each: outputs of one shape are sampled at the same positions)
+    host = {name: host_sample(a, DUMP_BYTES // len(outs), np.random.default_rng(0)) for name, a in outs.items()}
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+        for name, x in host.items():
+            assert x.dtype in (np.float32, np.float64), (name, x.dtype)
+            np.save(os.path.join(path, name + ".npy"), x)
 
 
 def time_workload(wl, steps, warmup, sampler=None):
@@ -666,6 +726,8 @@ def run_ours(args):
     clocks = sampler.stop()
     exact = wl.check()
     assert exact, "config %d: the timed result is wrong" % cfg
+    if args.dump_outputs:
+        dump_outputs(wl, args.dump_outputs, rank)
     value = wl.bytes_per_step * args.steps / tm["elapsed"] / 1e9
     roofline = roofline_entry(wl, tm, W, cfg)
     e2e = None

@@ -55,5 +55,5 @@ _cabi.launch_count = lambda: cnt[0]
 _cabi.reset_launch_count = lambda: cnt.__setitem__(0, 0)
 import bench
 sys.argv = ["bench.py", "--gpus", os.environ.get("WORLD_SIZE", "1"), "--steps", "3", "--warmup", "3", "--n", "200000", "--scale", "0.03125", "--no-cpu",
-            "--extra-steps", "2", "--e2e-steps", "2"]
+            "--extra-steps", "2", "--e2e-steps", "2"] + sys.argv[1:]
 bench.main()

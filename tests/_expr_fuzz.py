@@ -147,7 +147,9 @@ def trig_mask_program(np, seed, n_actions=36):
         elif k == 2:
             x = f(); s = np.sin(x); y = f(); u = y * 2.0; y[:, :] = np.cos(x); put(F, u + s)   # the pair's second half overwrites y
         elif k == 3:
-            put(F, np.sqrt(abs(f())) + np.exp(np.minimum(f(), 2.0)))
+            # (+ 0.25 keeps sqrt's slope at most 1: an operand such as sin(x)**2 + cos(x)**2 - 1.0 is rounding noise, and
+            # sqrt(abs(.)) of it would turn one ulp of another sin / cos implementation into 1e-8)
+            put(F, np.sqrt(abs(f()) + 0.25) + np.exp(np.minimum(f(), 2.0)))
         elif k == 4:
             x = f(); m = g() > 0.0; x[m] = 0.5                 # boolean-mask assignment (mask from exact data: no comparison
                                                                # can fall differently on another sin / cos implementation)
